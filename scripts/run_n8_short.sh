@@ -1,4 +1,4 @@
-cd /root/repo
+cd "$(dirname "$0")/.."
 mkdir -p gpurun_out
 export DJ_TEST_LIGHT=1
 TRP="python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1"

@@ -48,6 +48,42 @@ def test_bench_reference_arm_under_torchrun_prints_one_line(monkeypatch):
     assert d["e2e"]["h2d_bytes_per_step"] == 0
 
 
+def test_bench_dump_outputs_is_independent_of_row_order(oracle, tmp_path):
+    """--dump-outputs samples the joined rows by content (the probe row id) and sorts them, so two runs that return
+    the same row multiset in different orders dump identical files, and every value survives float64 exactly.
+    The table is larger than the sample, so the dump holds a strict subset of the joined rows.  Rows whose probe
+    payload is not a probe row id (a corrupt result) are left out instead of failing the dump."""
+    import numpy as np
+    import torch
+
+    import bench
+
+    n = 3_000_000
+    assert n > bench.DUMP_PROBE_ROWS
+    g = oracle.gen_params(n, n, 0.3, 2 * n, True)
+    bk, bp, _ = oracle.generate_rows(g, 0, 0, 0, n)
+    pk, pp, hits = oracle.generate_rows(g, 1, 0, 0, n)
+    n_out, cols = oracle.inner_join(bk, bp, pk, pp)
+    bad = [np.array([7, 7], np.int64), np.array([1, 2], np.int64), np.array([7, 7], np.int64),
+           np.array([-1, n], np.int64)]
+    dumps = []
+    for seed, extra in ((1, False), (2, False), (3, True)):
+        perm = np.random.default_rng(seed).permutation(n_out)
+        rows = [np.concatenate([c[perm], b]) if extra else c[perm] for c, b in zip(cols, bad)]
+        bench.dump_outputs(str(tmp_path / str(seed)), [torch.from_numpy(c) for c in rows], n_out, n, 1, 0)
+        dumps.append({f: np.load(tmp_path / str(seed) / f"{f}.npy") for f in ("n_out",) + bench.DUMP_COLS})
+    for d in dumps[1:]:
+        for f, a in dumps[0].items():
+            assert a.dtype == np.float64 and np.array_equal(a, d[f]), f
+    assert dumps[0]["n_out"][0] == n_out == hits
+    ids = np.random.default_rng(bench.DUMP_SEED).choice(n, bench.DUMP_PROBE_ROWS, replace=False)
+    keep = np.isin(cols[3], ids)
+    assert 0 < keep.sum() < n_out
+    want = oracle.sort_rows(*[c[keep] for c in cols][::-1])[::-1]  # right_payload is the primary sort key
+    for f, w in zip(bench.DUMP_COLS, want):
+        assert np.array_equal(dumps[0][f], w.astype(np.float64)), f
+
+
 def test_bench_import_does_not_pin_openmp():
     """Regression: OMP_PROC_BIND / OMP_PLACES exported at import time pinned EVERY rank's main thread to core 0
     (libgomp binds the initial thread): 105 instead of 9.5 ms/step at N=8.  They may only be set by the

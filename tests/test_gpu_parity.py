@@ -175,6 +175,32 @@ def test_full_size_properties_100m(dj, oracle):
     assert n2 == hits and dj.multiset_checksum4(cols2[2], cols2[3], cols2[0], cols2[1]) == ck
 
 
+def test_bench_steps_and_dump_outputs(dj, tmp_path):
+    """bench.py at a small size: --steps sets how many steps are timed in the HBM-resident and the e2e window
+    (the kernel launches of each scale with it, --warmup 0 included), the timed result passes parity, and
+    --dump-outputs writes that result's row count."""
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    runs = {}
+    for steps in (1, 3):
+        out = tmp_path / f"dump{steps}"
+        r = subprocess.run([sys.executable, "bench.py", "--gpus", "1", "--steps", str(steps), "--warmup", "0",
+                            "--rows", "2000000", "--no-cpu", "--dump-outputs", str(out)], cwd=root,
+                           capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-2000:]
+        d = json.loads([line for line in r.stdout.splitlines() if line.startswith("{")][-1])
+        assert d["steps"] == steps and d["e2e"]["steps"] == steps
+        assert d["parity"]["rows_ok"] and d["parity"]["checksum_ok"]
+        assert np.load(out / "n_out.npy")[0] == d["output_rows"] > 0
+        runs[steps] = (d["gpu_launches"], d["e2e"]["gpu_launches"], {f.name: np.load(f) for f in out.iterdir()})
+    assert runs[3][0] == 3 * runs[1][0] > 0
+    assert runs[3][1] == 3 * runs[1][1] > 0
+    for f, a in runs[1][2].items():
+        assert a.dtype == np.float64 and np.array_equal(a, runs[3][2][f]), f
+
+
 def test_multi_gpu_parity_under_torchrun():
     """N >= 2 ranks over NCCL (skipped on a single-GPU box): tests/test_multi_gpu.py under torchrun."""
     import socket
