@@ -64,7 +64,8 @@ ABI_SYMBOLS = [
     "dj_version", "dj_last_error", "dj_kernel_launch_count", "dj_profile_enable", "dj_profile_read",
     "dj_partition_ids_i64",
     "dj_hash_partition_workspace_bytes", "dj_hash_partition_i64", "dj_inner_join_workspace_bytes",
-    "dj_inner_join_i64", "dj_generate_build_bitmap", "dj_generate_rows_i64", "dj_multiset_checksum4",
+    "dj_inner_join_i64", "dj_hash_partition_cols_workspace_bytes", "dj_hash_partition_cols",
+    "dj_inner_join_cols_workspace_bytes", "dj_inner_join_cols", "dj_generate_build_bitmap", "dj_generate_rows_i64", "dj_multiset_checksum4",
     "dj_comm_unique_id", "dj_comm_create", "dj_comm_destroy", "dj_comm_release_workspace", "dj_comm_nccl_handle",
     "dj_comm_rank",
     "dj_comm_size",
@@ -100,6 +101,15 @@ def lib() -> C.CDLL:
     L.dj_inner_join_workspace_bytes.restype = sz
     L.dj_inner_join_workspace_bytes.argtypes = [i64, i64]
     L.dj_inner_join_i64.argtypes = [vp, vp, i64, vp, vp, i64, vp, vp, vp, vp, i64, vp, vp, sz, vp]
+    pvp, pint = C.POINTER(vp), C.POINTER(C.c_int)
+    L.dj_hash_partition_cols_workspace_bytes.restype = sz
+    L.dj_hash_partition_cols_workspace_bytes.argtypes = [i64, C.c_int]
+    L.dj_hash_partition_cols.argtypes = [vp, pvp, pint, C.c_int, i64, C.c_int, u32, C.c_int, vp, pvp, vp, vp, sz,
+                                         vp]
+    L.dj_inner_join_cols_workspace_bytes.restype = sz
+    L.dj_inner_join_cols_workspace_bytes.argtypes = [i64, i64, i64]
+    L.dj_inner_join_cols.argtypes = [vp, pvp, pint, C.c_int, i64, vp, pvp, pint, C.c_int, i64, vp, pvp, vp, pvp, i64,
+                                     vp, vp, sz, vp]
     L.dj_generate_build_bitmap.argtypes = [C.POINTER(GenParams), C.c_int, vp, vp]
     L.dj_generate_rows_i64.argtypes = [C.POINTER(GenParams), C.c_int, C.c_int, i64, i64, vp, vp, vp, vp]
     L.dj_multiset_checksum4.argtypes = [vp, vp, vp, vp, i64, vp, vp]
@@ -214,6 +224,68 @@ def inner_join(bk, bp, pk, pp, capacity=None, ws=None):
         n = int(cnt.item())
         if n <= capacity:
             return tuple(o[:n] for o in outs), n
+        capacity = n  # exact retry, as dj_b200.h documents
+
+
+MAX_PAYLOAD_COLUMNS = 15  # DJ_MAX_PAYLOAD_COLUMNS
+
+
+def _cols_dev(cols):
+    """Payload columns of a wide table: contiguous CUDA tensors of any 4- or 8-byte dtype, moved bitwise."""
+    cols = list(cols)
+    for c in cols:
+        if not (c.is_cuda and c.is_contiguous() and c.dim() == 1 and c.element_size() in (4, 8)):
+            raise DjError("expected contiguous 1-D CUDA tensors with 4- or 8-byte elements")
+    return cols
+
+
+def _col_arrays(cols):
+    """(host array of device pointers, host array of widths) for the _cols ABI."""
+    vp = C.c_void_p
+    return (vp * max(len(cols), 1))(*[c.data_ptr() for c in cols]), \
+        (C.c_int * max(len(cols), 1))(*[c.element_size() for c in cols])
+
+
+def hash_partition_cols(keys, cols, nparts, seed=SEED_NVLINK, hash_id=HASH_MURMUR3):
+    """cudf::hash_partition of a wide table: an int64 key plus 0..15 payload columns of any 4- or 8-byte
+    dtype.  Returns (keys_out, [col_out...], offsets[nparts+1]); offsets equal hash_partition's."""
+    keys = _i64dev(keys)
+    cols = _cols_dev(cols)
+    n = keys.numel()
+    ko = torch.empty_like(keys)
+    cos = [torch.empty_like(c) for c in cols]
+    offsets = torch.empty(nparts + 1, dtype=torch.int64, device=keys.device)
+    ws = workspace(lib().dj_hash_partition_cols_workspace_bytes(n, nparts), keys.device)
+    pin, widths = _col_arrays(cols)
+    pout, _ = _col_arrays(cos)
+    _check(lib().dj_hash_partition_cols(_ptr(keys), pin, widths, len(cols), n, nparts, seed, hash_id, _ptr(ko), pout,
+                                        _ptr(offsets), _ptr(ws), ws.numel(), _stream()))
+    return ko, cos, offsets
+
+
+def inner_join_cols(bk, bcols, pk, pcols, capacity=None):
+    """cudf::inner_join of wide tables: int64 keys plus 0..15 payload columns per side of any 4- or 8-byte
+    dtype.  Returns ((build key, [build cols], probe key, [probe cols]) trimmed to n_out, n_out)."""
+    bk, pk = _i64dev(bk), _i64dev(pk)
+    bcols, pcols = _cols_dev(bcols), _cols_dev(pcols)
+    nb, np_ = bk.numel(), pk.numel()
+    if capacity is None:
+        capacity = max(np_, 1)
+    dev = bk.device
+    bin_, bw = _col_arrays(bcols)
+    pin, pw = _col_arrays(pcols)
+    while True:
+        bko, pko = (torch.empty(capacity, dtype=torch.int64, device=dev) for _ in range(2))
+        bout = [torch.empty(capacity, dtype=c.dtype, device=dev) for c in bcols]
+        pout = [torch.empty(capacity, dtype=c.dtype, device=dev) for c in pcols]
+        cnt = torch.zeros(1, dtype=torch.int64, device=dev)
+        ws = workspace(lib().dj_inner_join_cols_workspace_bytes(nb, np_, capacity), dev)  # grows with capacity
+        _check(lib().dj_inner_join_cols(_ptr(bk), bin_, bw, len(bcols), nb, _ptr(pk), pin, pw, len(pcols), np_,
+                                        _ptr(bko), _col_arrays(bout)[0], _ptr(pko), _col_arrays(pout)[0], capacity,
+                                        _ptr(cnt), _ptr(ws), ws.numel(), _stream()))
+        n = int(cnt.item())
+        if n <= capacity:
+            return (bko[:n], [c[:n] for c in bout], pko[:n], [c[:n] for c in pout]), n
         capacity = n  # exact retry, as dj_b200.h documents
 
 

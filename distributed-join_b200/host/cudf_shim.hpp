@@ -1,7 +1,7 @@
 // cudf_shim.hpp -- the small slice of the cuDF / RMM vocabulary that the reference's public
 // API and drivers are written against (SURVEY.md App. C), implemented over plain CUDA memory and
 // the dj_b200 C ABI.  Only what the hot path touches exists: fixed-width columns, non-owning
-// views, tables, hash_partition / inner_join / concatenate for INT64 columns.
+// views, tables, hash_partition / inner_join / concatenate for 4- and 8-byte columns.
 //
 // This is what lets benchmark/distributed_join.cu keep its source shape
 //   (cudf::table_view, std::unique_ptr<cudf::table>, cudf::hash_id::HASH_MURMUR3, rmm pool ...)
@@ -281,13 +281,21 @@ bool all_i64(table_view const& t);
 
 // cudf::hash_partition(table, {key column}, nparts, hash, seed) -> (partitioned table, offsets[nparts])
 // (call sites src/distributed_join.cpp:213-225, src/shuffle_on.cpp:59-60).  Fixed-width columns, one
-// key column, up to three further columns; runs dj_hash_partition_i64 on stream 0.
+// key column at any position.  A key plus 1..3 further columns runs dj_hash_partition_i64 (4-byte
+// columns widened as above); any other table -- a key alone or with up to DJ_MAX_PAYLOAD_COLUMNS
+// further columns -- runs dj_hash_partition_cols, which moves every non-key column at its own width
+// (only a 4-byte key is widened).  Both hash the same int64 key, so a row lands in the same partition
+// whichever path its table takes.  Stream 0.
 std::pair<std::unique_ptr<table>, std::vector<size_type>> hash_partition(
   table_view const& input, std::vector<size_type> const& columns_to_hash, int num_partitions,
   hash_id hash_function = hash_id::HASH_MURMUR3, uint32_t seed = DEFAULT_HASH_SEED);
 
 // cudf::inner_join(left, right, {0}, {0}) -> left columns ++ right columns
-// (src/distributed_join.cpp:79).  Two fixed-width columns per side; runs dj_inner_join_i64.
+// (src/distributed_join.cpp:79).  One key column per side at any position.  Two fixed-width columns
+// per side run dj_inner_join_i64; any other fixed-width tables (key + 0..DJ_MAX_PAYLOAD_COLUMNS
+// columns per side) run dj_inner_join_cols, which joins (key, row index) and gathers the other
+// columns at their own widths.  Builds on the smaller side; the output is all left columns ++ all
+// right columns in their original positions and types.
 std::unique_ptr<table> inner_join(table_view const& left, table_view const& right,
                                   std::vector<size_type> const& left_on,
                                   std::vector<size_type> const& right_on);

@@ -99,6 +99,48 @@ int dj_inner_join_i64(const int64_t* d_build_key, const int64_t* d_build_payload
                       void* d_workspace, size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------------------------
+ * Wide tables: an int64 key plus 0..DJ_MAX_PAYLOAD_COLUMNS fixed-width payload columns per
+ * side, each 4 or 8 bytes wide (h_elem_bytes[c]).  Columns are moved bitwise, so any 4- or
+ * 8-byte type works (int32, float, timestamps, double ...).  Both calls run the pipelines
+ * above on (key, row index) and then gather every payload column through the resulting row
+ * indices at its own width (late materialization), so the partition and join kernels move
+ * 16 bytes per row whatever the table's width.  h_cols / h_out_cols are HOST arrays of
+ * device pointers.  Arguments are checked before any CUDA call: a column count out of range,
+ * a width other than 4 or 8, or a null column / key pointer where rows are read or written
+ * returns DJ_ERR_ARG; a workspace below the matching *_workspace_bytes query returns
+ * DJ_ERR_WORKSPACE.  The workspace queries need no GPU.
+ */
+#define DJ_MAX_PAYLOAD_COLUMNS 15
+
+/* dj_hash_partition_cols -- cudf::hash_partition(table, {key}, nparts, hash, seed) for a wide
+ * table, with the contract of dj_hash_partition_i64: d_offsets (nparts+1 entries) is
+ * bit-identical to dj_hash_partition_i64's for the same keys, seed and nparts, so wide and
+ * 2-column tables partitioned with the same seed co-locate; order inside a partition is
+ * unspecified; every output row is one intact input row.  1 <= nparts <= 1024. */
+size_t dj_hash_partition_cols_workspace_bytes(int64_t nrows, int nparts);
+int dj_hash_partition_cols(const int64_t* d_key, const void* const* h_cols, const int* h_elem_bytes,
+                           int ncols, int64_t nrows, int nparts, uint32_t seed, int hash_id,
+                           int64_t* d_out_key, void* const* h_out_cols, int64_t* d_offsets,
+                           void* d_workspace, size_t workspace_bytes, void* stream);
+
+/* dj_inner_join_cols -- cudf::inner_join(left, right, {key}, {key}) for wide tables, with the
+ * contract of dj_inner_join_i64: multimap semantics; outputs are (build key, build columns,
+ * probe key, probe columns), each column at its input's width; at most out_capacity rows are
+ * written and *d_out_count always receives the exact cardinality, so a caller that
+ * under-allocated can retry with a larger output (and workspace: it grows with out_capacity);
+ * either side empty -> 0 rows.  No host synchronisation: the payload gathers read the count
+ * on the device. */
+size_t dj_inner_join_cols_workspace_bytes(int64_t nbuild, int64_t nprobe, int64_t out_capacity);
+int dj_inner_join_cols(const int64_t* d_build_key, const void* const* h_build_cols,
+                       const int* h_build_elem_bytes, int nbuild_cols, int64_t nbuild,
+                       const int64_t* d_probe_key, const void* const* h_probe_cols,
+                       const int* h_probe_elem_bytes, int nprobe_cols, int64_t nprobe,
+                       int64_t* d_out_build_key, void* const* h_out_build_cols,
+                       int64_t* d_out_probe_key, void* const* h_out_probe_cols,
+                       int64_t out_capacity, int64_t* d_out_count,
+                       void* d_workspace, size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------------------------
  * Input generator -- replaces generate_input_tables / generate_tables_distributed
  * (generate_dataset/generate_dataset.cuh:163-260, src/generate_table.cuh:155-272) with a
  * counter-based restatement (Philox4x32-10 + Feistel permutation) shared bit-for-bit with
